@@ -234,6 +234,18 @@ def cat_results(parts):
     return tuple(np.concatenate([p[i] for p in parts]) for i in range(3))
 
 
+def dump_outputs(path, result):
+    """The configs[2] answer of the last timed step (all datanodes' groups) as float64 .npy files.  The library returns
+    groups in hash-table order, so rows are put in group-key order: two builds then compare array by array."""
+    keys, aggs, nulls = result
+    order = np.lexsort(keys.T[::-1]) if keys.shape[1] else np.arange(len(keys))
+    os.makedirs(path, exist_ok=True)
+    arrays = {"o_orderdate": keys[order, 0], "count_star": aggs[order, 0].view(np.int64),
+              "sum_l_extendedprice": aggs[order, 1], "nulls": nulls[order]}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def phase_table(ctx, names, steps):
     out = {}
     for name in names:
@@ -352,6 +364,10 @@ def run_ours(args):
     nl_total = allsum(float(nl))
     checks = {"count_star_equals_lineitem_rows": int(count_total) == int(nl_total),
               "groups_this_node": int(len(keys))}
+    if args.dump_outputs:
+        parts = gather0(last)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, cat_results(parts))
 
     # ---- the other BASELINE configurations, same run, same tables (extras; the headline stays configs[2])
     extras = {}
@@ -773,7 +789,11 @@ def main():
     ap.add_argument("--no-unclustered", action="store_true", help="skip the row-permuted variant")
     ap.add_argument("--pages-gb", type=float, default=10.0, help="GB of heap pages pushed through the page loader (e2e_pages leg; 0 = skip)")
     ap.add_argument("--cpu-sample-orders", type=int, default=1_500_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline query's answer from the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     # stdout carries exactly one JSON line: anything a library prints on fd 1 meanwhile (NCCL's
